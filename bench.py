@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — flow-pairs/s of the hot path on synthetic frame streams (BASELINE.json: tvl1 @ 1920x1080).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload tvl1_1080p|...]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload tvl1_1080p|...] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input: `--pairs` (default 16)
 consecutive frame pairs of a seeded synthetic stream (17 gray frames), i.e. one call of the batch shape of
@@ -41,6 +41,8 @@ NWIN = 2  # distinct input windows of pairs+1 frames each, alternated between st
 # dram__bytes_read.sum + dram__bytes_write.sum per launch of the dominant kernel, from the committed `ncu --set full`
 # captures (scripts/ncu_traffic.py writes this file from the raw CSV pages under profiles/)
 NCU_TRAFFIC_FILE = os.path.join(ROOT, "profiles", "ncu_traffic.json")
+DUMP_MAX_BYTES = 64 << 20  # --dump-outputs: a larger batch of flows is written as a seeded sample of DUMP_SAMPLE flow vectors
+DUMP_SAMPLE = 1 << 22
 
 
 def ncu_traffic(workload, pairs_per_launch):
@@ -77,7 +79,14 @@ def parse():
     # the reference's per-batch chain minus decode / file IO: BGR frames -> gray -> resize -> flow -> quantise -> 2 JPEGs per pair
     ap.add_argument("--chain", action="store_true", help="chain mode: dfb_process_bgr_batch_host on BGR frames of --chain-src size")
     ap.add_argument("--chain-src", default="", help="WxH of the decoded BGR frames (default: the workload's size, i.e. no resize)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the flows the timed path returned in its last step (rank 0) to DIR/flow.npy, float32: [pairs,H,W,2] "
+                         "up to 64 MB, else the flow vectors at %d seeded (pair, y, x) positions in increasing order, [n,2]" % DUMP_SAMPLE)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.list or args.chain):
+        ap.error("--dump-outputs writes the flows of the default timed path; it does not apply to --impl reference, --list or --chain")
     if args.pairs <= 0:
         args.pairs = 63 if args.workload in ("tvl1_340x256", "tvl1_256") else 16
     return args
@@ -144,6 +153,19 @@ def load_peaks():
     if os.path.exists(p):
         return json.load(open(p)).get("hbm_gbs"), "measured (MEASURED_PEAKS.json hbm_gbs)"
     return 6650.0, "fallback (B200_PROFILING.md 6.65 TB/s)"
+
+
+def dump_flows(flows_dev, out_dir):
+    """--dump-outputs: the float32 flows [P,H,W,2] of a step as out_dir/flow.npy, or a fixed sample of them when larger than
+    DUMP_MAX_BYTES, so that two builds can be compared output for output on the same arguments."""
+    import numpy as np
+    import torch
+    f = flows_dev
+    if f.numel() * f.element_size() > DUMP_MAX_BYTES:
+        idx = np.sort(np.random.default_rng(0).integers(0, f.numel() // 2, DUMP_SAMPLE))
+        f = f.reshape(-1, 2)[torch.from_numpy(idx).to(f.device)]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "flow.npy"), f.cpu().numpy())
 
 
 def make_stream(W, H, n_frames, seed, rank):
@@ -543,6 +565,8 @@ def main():
     launches = int(shard.all_sum(c["kernel_launches"], dev))
     total_pairs = world * args.steps * P
     value = total_pairs / dt_dev_max
+    if args.dump_outputs and rank == 0:
+        dump_flows(flows_dev, args.dump_outputs)  # before the unfused-schedule and parity runs below overwrite flows_dev
 
     # ---------------- roofline of the dominant kernel (rank 0's GPU) --------------------------------------
     roof = None
